@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the unmodified reference extension (oracle/_ref)
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs as DIR/<name>.npy
 
 Metric (BASELINE.json): fwd+bwd Gaussians/s at 2M points, 1920x1280.
 A "step" is one pass of the render hot path over one view: rasterizer forward
@@ -45,7 +46,9 @@ import torch.distributed as dist
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline metric and its e2e line; the training-iteration and config 1-4 "
+                         "legs time their own fixed counts")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--points", type=int, default=2_000_000)
@@ -72,7 +75,31 @@ def parse():
                     help="skip the BASELINE config 1-4 legs (bench_configs.py, N == 1 only)")
     ap.add_argument("--configs", default="config1,config2,config3,config4",
                     help="which of the extra config legs to run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (images, radii, gradients) "
+                         "as DIR/<name>.npy, at most 64 MB in all, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def dump_outputs(out_dir, arrays, budget=64_000_000):
+    """Write each (name, tensor) of `arrays` as out_dir/<name>.npy in float32 (float64 stays float64).  Every array
+    gets an equal share of `budget` bytes; one that is larger is replaced by a fixed sample of its flattened elements
+    (positions drawn from a generator seeded by the name), so that runs with the same arguments sample the same
+    positions."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // max(len(arrays), 1) - 4096          # room for the .npy header
+    for name, x in arrays:
+        dt = torch.float64 if x.dtype == torch.float64 else torch.float32
+        x = x.detach()
+        k = share // (8 if dt == torch.float64 else 4)
+        if x.numel() > k:
+            idx = np.unique(np.random.default_rng(zlib.crc32(name.encode())).integers(0, x.numel(), k))
+            x = x.reshape(-1)[torch.from_numpy(idx).to(x.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), x.to(dt).cpu().numpy())
 
 
 class ClockSampler:
@@ -154,6 +181,7 @@ def load_impl(name):
 
 def main():
     a = parse()
+    torch.manual_seed(0)            # host-side random inputs (ground-truth images) are the same from run to run
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -262,6 +290,8 @@ def main():
             return flat
         return None
 
+    last = {}
+
     def step_resident():
         zero_grads()
         color, radii, depth = rast(means3D=t["means3D"], means2D=m2d, opacities=t["opacities"], shs=t["shs"],
@@ -269,6 +299,8 @@ def main():
                                    rotations=t["rotations"], cov3D_precomp=None)
         torch.autograd.backward([color, depth], [gc, gd])
         allreduce_grads()
+        if a.dump_outputs:
+            last.update(color=color, radii=radii, depth=depth)
         return radii
 
     # ---- host-driven end-to-end step -------------------------------------
@@ -357,6 +389,12 @@ def main():
     ms_res = timed(step_resident, a.steps, max(a.warmup, 3))
     ms_res_local = local_ms["last"]
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        # the gradients of the last timed step are still on the leaves.  N > 1: ours writes them into the reduced
+        # bucket, the reference arm reduces a concatenated copy, so there rank 0's own, unreduced gradients are written
+        dump_outputs(a.dump_outputs, [(k, last[k]) for k in ("color", "depth", "radii")] +
+                     [("grad_" + k, t[k].grad) for k in util.TENSOR_KEYS if t[k] is not None] +
+                     [("grad_means2D", m2d.grad)])
     ms_e2e = timed(step_e2e, a.steps, 3)
 
     radii = step_resident()
@@ -640,11 +678,16 @@ def main_fine(a, rank, world, local, dev):
             flat = torch.cat([v.grad.reshape(-1) for v in leaves if v.grad is not None])
             dist.all_reduce(flat)
 
+    last = {}
+
     def step_resident():
         for v in leaves:
             v.grad = None
-        loss_of(do_render(), img_d, dep_d, feat_d).backward()
+        out = do_render()
+        loss_of(out, img_d, dep_d, feat_d).backward()
         sync_grads()
+        if a.dump_outputs:
+            last.update(out)
 
     loss_host = torch.zeros(1).pin_memory()
 
@@ -682,6 +725,10 @@ def main_fine(a, rank, world, local, dev):
         sampler.start()
     ms_res = timed(step_resident, a.steps, max(a.warmup, 3))
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, [(k, last[k]) for k in ("render", "depth", "feat", "radii", "dx", "dshs")] +
+                     [("grad_viewspace_points", last["viewspace_points"].grad)] +
+                     [(f"grad_leaf{i:02d}", v.grad) for i, v in enumerate(leaves) if v.grad is not None])
     ms_e2e = timed(step_e2e, a.steps, 3)
     # ---- whole fine-stage training iteration (N == 1): render + every loss term of train.py:395-425 incl. SSIM and
     # the plane regularisers + backward + densify stats + Adam over Gaussians, planes and decoder ------------------

@@ -158,46 +158,35 @@ def test_densify_stats_matches_reference_golden(built_lib):
     assert np.array_equal(max_radii.cpu().numpy(), z["max_radii2D"])
 
 
+LOSS_CASES = [("ssim", (2, 3, 640, 960), 9), ("l1_depth", (2, 3, 640, 960), 10), ("l1_depth_odd", (1, 3, 37, 53), 10)]
+LOSS_SAMPLE = 1024
+
+
 def test_image_loss_matches_reference_functions_on_gpu(built_lib):
-    """Where oracle/_ref travels: the reference's own l1_loss / ssim / compute_depth (cuDNN depthwise convs)
-    on the same GPU, composed as train.py:395-419."""
-    import ref_ext
-    if not ref_ext.loss_utils_available():
-        pytest.skip("oracle/_ref/s3g_ref/utils/loss_utils.py not present (run oracle/build_ref.sh)")
-    lu = ref_ext.load_ref_loss_utils()
+    """The reference's own l1_loss / ssim / compute_depth (cuDNN depthwise convs, TF32 off) on the same GPU, composed
+    as train.py:395-419: tests/golden/ref_image_loss.npz holds its loss and, at fixed positions, its gradients
+    (tools/make_golden_refext.py)."""
     from s3gaussian_b200 import losses
-    img, gt, depth, gt_depth = [t.to(DEV) for t in mg.loss_inputs(2, 3, 640, 960, 9)]
-    x = img.clone().requires_grad_(True)
-    d = depth.clone().requires_grad_(True)
-    ours = losses.training_loss(x, gt, d, gt_depth)
-    ours.backward()
-    xr = img.clone().requires_grad_(True)
-    dr = depth.clone().requires_grad_(True)
-    prev = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False
-    try:
-        ref = lu.l1_loss(xr, gt) + 0.5 * lu.compute_depth("l2", dr, gt_depth) + 0.2 * (1.0 - lu.ssim(xr, gt))
-        ref.backward()
-    finally:
-        torch.backends.cudnn.allow_tf32 = prev
-    assert abs(ours.item() - ref.item()) < 1e-5
-    assert rel(x.grad, xr.grad) < 1e-4
-    assert rel(d.grad, dr.grad) < 1e-5
-    # lambda_dssim == 0 (train.py:418 does not evaluate SSIM then): the stencil-free kernels, odd sizes included
-    for shape in ((2, 3, 640, 960), (1, 3, 37, 53)):
-        img, gt, depth, gt_depth = [t.to(DEV) for t in mg.loss_inputs(*shape, 10)]
+    import util
+    z = util.load_golden(os.path.join(GOLD, "ref_image_loss.npz"))
+    for name, shape, seed in LOSS_CASES:
+        img, gt, depth, gt_depth = [t.to(DEV) for t in mg.loss_inputs(*shape, seed)]
         x = img.clone().requires_grad_(True)
         d = depth.clone().requires_grad_(True)
-        ours = losses.training_loss(x, gt, d, gt_depth, lambda_dssim=0.0, lambda_depth=0.5)
+        if name == "ssim":
+            ours = losses.training_loss(x, gt, d, gt_depth)
+            bars = (1e-5, 1e-4, 1e-5)
+        else:
+            # lambda_dssim == 0 (train.py:418 does not evaluate SSIM then): the stencil-free kernels, odd sizes included
+            ours = losses.training_loss(x, gt, d, gt_depth, lambda_dssim=0.0, lambda_depth=0.5)
+            bars = (1e-6, 1e-6, 1e-5)
         ours.backward()
-        xr = img.clone().requires_grad_(True)
-        dr = depth.clone().requires_grad_(True)
-        ref = lu.l1_loss(xr, gt) + 0.5 * lu.compute_depth("l2", dr, gt_depth)
-        ref.backward()
-        assert abs(ours.item() - ref.item()) < 1e-6, shape
-        assert rel(x.grad, xr.grad) < 1e-6 and rel(d.grad, dr.grad) < 1e-5, shape
-        l1, ss, dl2 = losses.image_loss_terms(x, gt, d, gt_depth, with_ssim=False)
-        assert float(ss) == 0.0
+        assert abs(ours.item() - float(z[name + "/loss"])) < bars[0], name
+        assert util.relerr_sampled(x.grad, z[name + "/gx_s"], z[name + "/gx_max"], LOSS_SAMPLE) < bars[1], name
+        assert util.relerr_sampled(d.grad, z[name + "/gd_s"], z[name + "/gd_max"], LOSS_SAMPLE) < bars[2], name
+        if name != "ssim":
+            l1, ss, dl2 = losses.image_loss_terms(x, gt, d, gt_depth, with_ssim=False)
+            assert float(ss) == 0.0
 
 
 def test_plane_regulation_matches_reference_golden(built_lib):
@@ -252,12 +241,14 @@ def test_plane_regulation_full_size_and_adam_on_channels_last_planes(built_lib):
 
 
 # ---- densify / prune against the reference's own methods ---------------------------------------
-def _pair_of_models(P, seed):
-    """Our GaussianModel and the reference's method bodies over identical tensors, optimizer state and
-    densification statistics."""
-    import ref_ext
+class _Params:
+    """Stand-in for the reference model in _pair_of_models when only the optimizer set-up is needed."""
+
+
+def _pair_of_models(P, seed, twin_cls=_Params):
+    """Our GaussianModel and a twin of class twin_cls (tools/make_golden_refext.py passes the reference's
+    GaussianModel method bodies) over identical tensors, optimizer state and densification statistics."""
     from s3gaussian_b200.gaussian_model import GaussianModel, default_optimization_params, PARAM_GROUPS, _ATTR
-    Ref = ref_ext.load_ref_gaussian_model_class()
     g = torch.Generator(device=DEV).manual_seed(seed)
     r = lambda *s: torch.randn(*s, device=DEV, generator=g)
     xyz = r(P, 3) * 10
@@ -265,14 +256,14 @@ def _pair_of_models(P, seed):
     ours = GaussianModel(3).create_from_tensors(xyz, r(P, 1, 3), r(P, 15, 3) * 0.1, scaling, r(P, 4), r(P, 1) * 2)
     opt_args = default_optimization_params()
     ours.training_setup(opt_args)
-    ref = Ref()
+    ref = twin_cls()
     for name in PARAM_GROUPS:
         setattr(ref, _ATTR[name], torch.nn.Parameter(getattr(ours, _ATTR[name]).detach().clone().requires_grad_(True)))
     ref.percent_dense = opt_args.percent_dense
     ref._deformation_table = torch.ones(P, dtype=torch.bool, device=DEV)
     ref.optimizer = torch.optim.Adam([{"params": [getattr(ref, _ATTR[n])], "lr": gr["lr"], "name": n}
                                       for n, gr in ((n, ours._group(n)) for n in PARAM_GROUPS)], lr=0.0, eps=1e-15)
-    # two optimizer steps on the reference, then copy its state into ours bit for bit
+    # two optimizer steps on the twin, then copy its state into ours bit for bit
     for _ in range(2):
         for n in PARAM_GROUPS:
             p = getattr(ref, _ATTR[n])
@@ -294,68 +285,80 @@ def _pair_of_models(P, seed):
     return ours, ref
 
 
-def _assert_same_state(ours, ref, what):
+def state_record(m):
+    """digest of every parameter, its Adam moments and step, and the densification statistics of model m (ours or
+    the reference's): what the densify / prune / reset steps are compared by"""
+    import util
     from s3gaussian_b200.gaussian_model import PARAM_GROUPS, _ATTR
+    rec = {}
     for n in PARAM_GROUPS:
-        po, pr = getattr(ours, _ATTR[n]), getattr(ref, _ATTR[n])
-        assert po.shape == pr.shape, (what, n, po.shape, pr.shape)
-        assert torch.equal(po.data, pr.data), (what, n)
-        so, sr = ours.optimizer.state.get(po), ref.optimizer.state.get(pr)
-        assert (so is None) == (sr is None), (what, n)
-        if so is not None:
-            assert torch.equal(so["exp_avg"], sr["exp_avg"]) and torch.equal(so["exp_avg_sq"], sr["exp_avg_sq"]), (what, n)
-            assert float(so["step"]) == float(sr["step"])
-        assert ours._group(n)["params"][0] is po
+        p = getattr(m, _ATTR[n])
+        st = m.optimizer.state.get(p)
+        rec[n] = util.digest(p.data) + str(tuple(p.shape))
+        rec[n + ".adam"] = "none" if st is None else \
+            util.digest(st["exp_avg"]) + util.digest(st["exp_avg_sq"]) + str(float(st["step"]))
     for a in ("xyz_gradient_accum", "denom", "max_radii2D", "_deformation_accum", "_deformation_table"):
-        assert torch.equal(getattr(ours, a), getattr(ref, a)), (what, a)
+        rec[a] = util.digest(getattr(m, a))
+    return rec
+
+
+def _assert_same_state(ours, z, what):
+    from s3gaussian_b200.gaussian_model import PARAM_GROUPS, _ATTR
+    for k, v in state_record(ours).items():
+        assert v == str(z[f"{what}/{k}"]), (what, k)
+    for n in PARAM_GROUPS:
+        assert ours._group(n)["params"][0] is getattr(ours, _ATTR[n])
+
+
+DENSIFY_SAMPLE = 512
 
 
 def test_densify_prune_reset_match_reference_methods(built_lib):
-    import ref_ext
-    if not ref_ext.gaussian_model_available():
-        pytest.skip("oracle/_ref/s3g_ref/scene/gaussian_model.py not present (run oracle/build_ref.sh)")
+    """Our densify / stats / prune / reset_opacity / Adam step against the reference's own GaussianModel methods run on
+    the same state: tests/golden/ref_densify.npz holds the reference's state after each step (digests, bit for bit)
+    and its parameters after the last Adam step (sampled) (tools/make_golden_refext.py)."""
+    import util
+    from s3gaussian_b200.gaussian_model import PARAM_GROUPS, _ATTR
+    z = util.load_golden(os.path.join(GOLD, "ref_densify.npz"))
     P = 50000
-    ours, ref = _pair_of_models(P, 7)
+    ours, _ = _pair_of_models(P, 7)
     extent = 20.0
-    # densify (clone + split), identical generator state for the torch.normal inside densify_and_split
+    # densify (clone + split), the generator state the reference saw for the torch.normal inside densify_and_split
     torch.manual_seed(123)
     ours.densify(0.0002, 0.005, extent, None)
-    torch.manual_seed(123)
-    ref.densify(0.0002, 0.005, extent, None, 5, 5, None, None, None)
     assert ours._xyz.shape[0] > P                      # the case is not degenerate
-    _assert_same_state(ours, ref, "densify")
+    _assert_same_state(ours, z, "densify")
     n1 = ours._xyz.shape[0]
     # statistics for the next round (ours: fused kernel; reference: its own method + train.py:490)
     g = torch.Generator(device=DEV).manual_seed(9)
     radii = torch.randint(0, 45, (n1,), device=DEV, generator=g, dtype=torch.int32)
     radii[torch.rand(n1, device=DEV, generator=g) < 0.3] = 0
     vgrad = torch.randn(n1, 3, device=DEV, generator=g) * 1e-3
+    acc = ours.xyz_gradient_accum.clone()
     ours.densification_step(vgrad, radii)
+    assert util.digest(ours.max_radii2D) == str(z["stats/max_radii2D"]) and util.digest(ours.denom) == str(z["stats/denom"])
+    # the reference's accumulation (add_densification_stats, one torch statement) on the same device: bit for bit
+    # what it stored; ours within 1e-6 (the fused kernel's norm differs in the last ulp), then re-synced for bit tests
     vis = radii > 0
-    ref.max_radii2D[vis] = torch.max(ref.max_radii2D[vis], radii[vis])
-    ref.add_densification_stats(vgrad, vis)
-    assert torch.equal(ours.max_radii2D, ref.max_radii2D) and torch.equal(ours.denom, ref.denom)
-    assert rel(ours.xyz_gradient_accum, ref.xyz_gradient_accum) < 1e-6
-    ours.xyz_gradient_accum = ref.xyz_gradient_accum.clone()       # 1-ulp differences of the norm: re-sync for bit tests
+    acc[vis] += torch.norm(vgrad[vis, :2], dim=-1, keepdim=True)
+    assert util.digest(acc) == str(z["stats/xyz_gradient_accum"])
+    assert rel(ours.xyz_gradient_accum, acc) < 1e-6
+    ours.xyz_gradient_accum = acc
     # prune with a screen-size limit (all three criteria)
     ours.prune(0.0002, 0.005, extent, 20)
-    ref.prune(0.0002, 0.005, extent, 20)
     assert ours._xyz.shape[0] < n1
-    _assert_same_state(ours, ref, "prune")
+    _assert_same_state(ours, z, "prune")
     # opacity reset: values, zeroed moments, kept step
     ours.reset_opacity()
-    ref.reset_opacity()
-    _assert_same_state(ours, ref, "reset_opacity")
+    _assert_same_state(ours, z, "reset_opacity")
     # an optimizer step still works on the rebuilt parameters and matches torch.optim.Adam
-    from s3gaussian_b200.gaussian_model import PARAM_GROUPS, _ATTR
     for n in PARAM_GROUPS:
-        po, pr = getattr(ours, _ATTR[n]), getattr(ref, _ATTR[n])
-        gr = torch.randn(po.shape, device=DEV, generator=g) * 0.01
-        po.grad, pr.grad = gr.clone(), gr.clone()
+        po = getattr(ours, _ATTR[n])
+        po.grad = torch.randn(po.shape, device=DEV, generator=g) * 0.01
     ours.optimizer.step()
-    ref.optimizer.step()
     for n in PARAM_GROUPS:
-        assert rel(getattr(ours, _ATTR[n]), getattr(ref, _ATTR[n])) < 2e-6, n
+        e = util.relerr_sampled(getattr(ours, _ATTR[n]), z[f"adam/{n}_s"], z[f"adam/{n}_max"], DENSIFY_SAMPLE)
+        assert e < 2e-6, (n, e)
     # split with nothing selected returns without touching anything (gaussian_model.py:507-508)
     before = ours._xyz.data_ptr()
     ours.densify_and_split(torch.zeros(ours._xyz.shape[0], 1, device=DEV), 1.0, extent)

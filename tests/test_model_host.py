@@ -1,15 +1,18 @@
 """Host-side (CPU) checks of GaussianModel against the reference's own method bodies: learning-rate schedule
-(scene/gaussian_model.py:203-218) taken from oracle/_ref with ast and executed unmodified."""
-import ast
+(scene/gaussian_model.py:203-218), taken from oracle/_ref with ast and executed unmodified by
+tools/make_golden_refext.py; its results are tests/golden/ref_lr_schedule.npz."""
 import os
-import types
 from argparse import Namespace
 
-import pytest
+import numpy as np
 import torch
 import torch.nn as nn
 
-import ref_ext
+import util
+
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+ITERATIONS = (1, 2, 500, 7000, 19999, 20000, 30000)
 
 OPT = Namespace(percent_dense=0.01, position_lr_init=0.00016, position_lr_final=0.0000016, position_lr_delay_mult=0.01,
                 position_lr_max_steps=20000, deformation_lr_init=0.000016, deformation_lr_final=0.0000016,
@@ -41,43 +44,20 @@ def _our_model():
     return m
 
 
-def _ref_functions():
-    base = os.path.join(ref_ext.REF_DIR, "s3g_ref")
-    ns = {"torch": torch, "nn": nn}
-    import numpy as np
-    ns["np"] = np
-
-    def grab(path, names):
-        for node in ast.walk(ast.parse(open(path).read())):
-            if isinstance(node, ast.FunctionDef) and node.name in names:
-                exec(compile(ast.Module(body=[node], type_ignores=[]), path, "exec"), ns)
-    grab(os.path.join(base, "utils", "general_utils.py"), {"get_expon_lr_func"})
-    grab(os.path.join(base, "scene", "gaussian_model.py"), {"update_learning_rate"})
-    return ns
-
-
-@pytest.mark.skipif(not ref_ext.gaussian_model_available(), reason="oracle/_ref/s3g_ref not present")
 def test_learning_rates_follow_the_reference_schedule():
-    ns = _ref_functions()
+    """tests/golden/ref_lr_schedule.npz: the reference's update_learning_rate over the same groups
+    (tools/make_golden_refext.py)."""
+    z = util.load_golden(os.path.join(GOLD, "ref_lr_schedule.npz"))
     m = _our_model()
     s = m.spatial_lr_scale
-    f = ns["get_expon_lr_func"]
-    ref = types.SimpleNamespace(
-        optimizer=types.SimpleNamespace(param_groups=[dict(g) for g in m.optimizer.param_groups]),
-        xyz_scheduler_args=f(lr_init=OPT.position_lr_init * s, lr_final=OPT.position_lr_final * s,
-                             lr_delay_mult=OPT.position_lr_delay_mult, max_steps=OPT.position_lr_max_steps),
-        deformation_scheduler_args=f(lr_init=OPT.deformation_lr_init * s, lr_final=OPT.deformation_lr_final * s,
-                                     lr_delay_mult=OPT.deformation_lr_delay_mult, max_steps=OPT.position_lr_max_steps),
-        grid_scheduler_args=f(lr_init=OPT.grid_lr_init * s, lr_final=OPT.grid_lr_final * s,
-                              lr_delay_mult=OPT.deformation_lr_delay_mult, max_steps=OPT.position_lr_max_steps))
     names = [g["name"] for g in m.optimizer.param_groups]
     assert names == ["xyz", "deformation", "grid", "f_dc", "f_rest", "opacity", "scaling", "rotation"]
-    for it in (1, 2, 500, 7000, 19999, 20000, 30000):
-        lr_ref = ns["update_learning_rate"](ref, it)
+    assert names == list(z["group_names"]) and tuple(z["iterations"]) == ITERATIONS
+    for i, it in enumerate(ITERATIONS):
         lr_ours = m.update_learning_rate(it)
-        assert lr_ours == lr_ref
-        for go, gr in zip(m.optimizer.param_groups, ref.optimizer.param_groups):
-            assert go["lr"] == gr["lr"], (it, go["name"])
+        assert lr_ours == z["lr"][i]
+        for go, lr_ref in zip(m.optimizer.param_groups, z["group_lr"][i]):
+            assert go["lr"] == lr_ref, (it, go["name"])
     d = {g["name"]: g["lr"] for g in m.optimizer.param_groups}
     assert abs(d["deformation"] - OPT.deformation_lr_final * s) < 1e-12      # decayed 1.6e-5 -> 1.6e-6 (x scale)
 

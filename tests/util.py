@@ -163,6 +163,95 @@ def grad_atol(ref_run_a, ref_run_b, floor_of_max=1e-6):
     return max(4.0 * float(np.abs(a - b).max()), floor_of_max * float(np.abs(a).max()))
 
 
+def _np(a):
+    return a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+
+
+def digest(a):
+    """sha256 of an array's bytes: stored in place of a large array that a test compares bit for bit."""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(_np(a)).tobytes()).hexdigest()
+
+
+def sample(a, k=256, seed=0, where=None):
+    """k elements of the flattened array at positions fixed by (size, k, seed): stored in place of a large float array
+    so that a test compares the same positions of its own result.  `where` (a mask of a's shape, e.g. the rows of
+    visible Gaussians, which both sides must agree on) restricts the draw to the positions it marks."""
+    a = _np(a).reshape(-1)
+    pos = np.arange(a.size) if where is None else np.flatnonzero(_np(where).reshape(-1))
+    if pos.size <= k:
+        return a[pos].copy()
+    return a[pos[np.sort(np.random.default_rng(seed).choice(pos.size, k, replace=False))]]
+
+
+def rows_mask(rows, shape):
+    """bool mask of `shape` marking every element of the rows (first axis) where `rows` is true"""
+    rows = _np(rows).astype(bool)
+    return np.broadcast_to(rows.reshape((-1,) + (1,) * (len(shape) - 1)), shape)
+
+
+def save_golden(path, record):
+    """Write a dict of arrays, numbers and strings as one .npz: an index (JSON) and one flat array per dtype.  A
+    record of hundreds of small entries would otherwise spend more on per-entry headers than on its values."""
+    import json
+    index, flat = {}, {}
+    for k, v in record.items():
+        if isinstance(v, str):
+            index[k] = v
+            continue
+        a = np.asarray(v)
+        key = a.dtype.str
+        off = sum(x.size for x in flat.setdefault(key, []))
+        flat[key].append(a.reshape(-1))
+        index[k] = [key, off, list(a.shape)]
+    np.savez_compressed(path, index=np.frombuffer(json.dumps(index).encode(), np.uint8),
+                        **{"d" + k.replace("<", "l").replace(">", "b").replace("|", "n"): np.concatenate(v)
+                           for k, v in flat.items()})
+
+
+def load_golden(path):
+    """dict of what save_golden() stored: strings as str, everything else as numpy arrays of the stored shape"""
+    import json
+    z = np.load(path)
+    index = json.loads(z["index"].tobytes().decode())
+    flat = {k: z[k] for k in z.files if k != "index"}
+    out = {}
+    for k, v in index.items():
+        if isinstance(v, str):
+            out[k] = v
+        else:
+            key, off, shape = v
+            n = int(np.prod(shape)) if shape else 1
+            out[k] = flat["d" + key.replace("<", "l").replace(">", "b").replace("|", "n")][off:off + n].reshape(shape)
+    return out
+
+
+def fill_uncovered(net, state, seed=6):
+    """Draw the parameters of `net` that the seeded `state` does not cover (time net, static_mlp) from a generator of
+    their own, in name order, so that the reference's network and ours get the same weights."""
+    g = torch.Generator().manual_seed(seed)
+    with torch.no_grad():
+        for k, p in sorted(net.named_parameters()):
+            if k not in state:
+                p.copy_(torch.randn(p.shape, generator=g) * 0.1)
+    return net
+
+
+def pick(a, k, seed=0):
+    """int32 positions of up to k nonzero elements of the flattened array: stored with the values there when the two
+    sides may disagree on which elements are zero"""
+    nz = np.flatnonzero(_np(a).reshape(-1))
+    if nz.size > k:
+        nz = nz[np.sort(np.random.default_rng(seed).choice(nz.size, k, replace=False))]
+    return nz.astype(np.int32)
+
+
+def relerr_sampled(ours, ref_sample, ref_absmax, k=256, seed=0, where=None):
+    """relerr() restricted to the stored sample positions, normalised by the full reference tensor's max."""
+    s = sample(ours, k, seed, where).astype(np.float64)
+    return float(np.abs(s - ref_sample).max() / (float(ref_absmax) + 1e-30)) if s.size else 0.0
+
+
 def seeded_grads(d, seed=1):
     g = torch.Generator().manual_seed(seed)
     return (torch.randn(3, d["H"], d["W"], generator=g), torch.randn(1, d["H"], d["W"], generator=g))
